@@ -447,7 +447,8 @@ def load_peaks():
 
 def timed_region(pipe, inputs, steps, warmup, host: bool, world: int, per_step: int = 1):
     """W warm-up steps, then EXACTLY K steps bracketed by barrier + synchronize; device-side events.  A step submits `per_step`
-    batches (1 in weak scaling; this rank's share of the host batch in strong scaling)."""
+    batches (1 in weak scaling; this rank's share of the host batch in strong scaling).  Returns (ms, wall seconds, the
+    pipeline slot of the last batch)."""
     import torch.distributed as dist
 
     submit = pipe.submit_host if host else pipe.submit_device
@@ -466,7 +467,7 @@ def timed_region(pipe, inputs, steps, warmup, host: bool, world: int, per_step: 
     pipe.fork(main)
     t0 = time.perf_counter()
     for _ in range(steps * per_step):
-        submit(inputs[k % len(inputs)])
+        last = submit(inputs[k % len(inputs)])
         k += 1
     pipe.join(main)
     e1.record(main)
@@ -478,7 +479,21 @@ def timed_region(pipe, inputs, steps, warmup, host: bool, world: int, per_step: 
 
     # the only communication of the path: SUM of scenes, MAX of the device-timed milliseconds (spsnet_b200/sharding.py)
     _, ms = sharding.reduce_report(BATCH * steps * per_step, e0.elapsed_time(e1), device="cuda")
-    return ms, wall
+    return ms, wall, last
+
+
+def dump_outputs(outs, out_dir, budget=64 << 20):
+    """The arrays a caller of the timed path receives, as <name>.npy: floats in float32, integers in float64 (exact).  An
+    array above its share of `budget` keeps a fixed, seeded sample of its rows, so two builds compare output for output."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = budget // max(len(outs), 1)
+    for k, v in outs.items():
+        a = v.float().numpy() if v.is_floating_point() else v.numpy().astype(np.float64)
+        if a.nbytes > share:
+            keep = max(1, share * a.shape[0] // a.nbytes)
+            a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))]
+        np.save(out_dir / f"{k}.npy", np.ascontiguousarray(a))
 
 
 class EagerRef:
@@ -653,6 +668,9 @@ def parse_args():
                     "this pool two cores per rank starve the CUDA helper threads: e2e 70.6k vs 78.2k scenes/s at N = 8, profiles/r02_*)")
     ap.add_argument("--out16", action="store_true", help="e2e: return centre features as fp16 (halves the D2H bytes; opt-in, default fp32 like the reference)")
     ap.add_argument("--timeline", action="store_true", help="e2e: CUDA-event timeline of H2D / forward / D2H per step (rank 0), printed in `e2e.timeline`")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="--impl ours: after the timed steps, write what the last timed step "
+                    "returned as DIR/<name>.npy (float32 / float64; a fixed, seeded sample of rows where the outputs exceed 64 MB); "
+                    "with several ranks, rank 0's batch")
     ap.add_argument("--workload", default="kitti", choices=sorted(WORKLOADS), help="kitti = BASELINE.json configs[1] (headline)")
     return ap.parse_args()
 
@@ -766,6 +784,8 @@ def main():
     rank, world, local = dist_env()
     args.warmup = max(args.warmup, 3)
 
+    if args.dump_outputs and args.impl != "ours":
+        raise SystemExit("bench.py: --dump-outputs writes the outputs of --impl ours only")
     if args.verify_only:
         return run_verify_only(args)
     if args.impl == "reference-cpu" or (args.impl == "reference" and not torch.cuda.is_available()):
@@ -814,9 +834,11 @@ def main():
     pipe.prepare(dev_pool[0])
     sampler = ClockSampler(local, enabled=rank == 0)   # one nvidia-smi poller per job, not one per rank (8 pollers contend for the driver)
     sampler.start()
-    ms, wall = timed_region(pipe, dev_pool, args.steps, args.warmup, host=False, world=world, per_step=per_step)
+    ms, wall, last = timed_region(pipe, dev_pool, args.steps, args.warmup, host=False, world=world, per_step=per_step)
+    # the slot's static outputs are overwritten by the next region: keep the last timed step's on the host
+    dumped = {k: v.cpu() for k, v in pipe.slots[last].outs.items()} if args.dump_outputs else None
     pipe.reset_timeline()
-    ms_e2e, _ = timed_region(pipe, host_pool, args.steps, args.warmup, host=True, world=world, per_step=per_step)
+    ms_e2e, _, _ = timed_region(pipe, host_pool, args.steps, args.warmup, host=True, world=world, per_step=per_step)
     clocks = sampler.stop()
     scenes_total = world * BATCH * args.steps * per_step
     value = scenes_total / (ms / 1e3)
@@ -840,8 +862,8 @@ def main():
         pipe1 = BackbonePipeline(net, BATCH, NPTS, NCOLS, depth=1, use_graph=not args.no_graph, extra_inputs=extra_inputs("cuda"), outputs=outputs)
         pipe1.prepare(dev_pool[0])
         s1 = max(8, min(args.steps, 32))
-        ms1, _ = timed_region(pipe1, dev_pool, s1, 3, host=False, world=world)
-        ms1h, _ = timed_region(pipe1, host_pool, s1, 3, host=True, world=world)
+        ms1, _, _ = timed_region(pipe1, dev_pool, s1, 3, host=False, world=world)
+        ms1h, _, _ = timed_region(pipe1, host_pool, s1, 3, host=True, world=world)
         line["depth1"] = {"value": world * BATCH * s1 / (ms1 / 1e3), "ms_per_step": ms1 / s1, "steps": s1, "unit": UNIT,
                           "e2e": world * BATCH * s1 / (ms1h / 1e3),
                           "note": "same workload with ONE batch in flight (pipeline_depth 1): ms_per_step here is the latency of a batch"}
@@ -860,6 +882,8 @@ def main():
         except Exception as e:  # pragma: no cover
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": f"failed: {e}"}
     line["config"] = cfg
+    if dumped is not None and rank == 0:
+        dump_outputs(dumped, args.dump_outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -888,8 +912,8 @@ def run_reference_gpu(args, rank, world, local, line, cfg):
     pipe.sync()
     sampler = ClockSampler(local, enabled=rank == 0)
     sampler.start()
-    ms, _ = timed_region(pipe, dev_pool, args.steps, args.warmup, host=False, world=world, per_step=per_step)
-    ms_e2e, _ = timed_region(pipe, host_pool, args.steps, args.warmup, host=True, world=world, per_step=per_step)
+    ms, _, _ = timed_region(pipe, dev_pool, args.steps, args.warmup, host=False, world=world, per_step=per_step)
+    ms_e2e, _, _ = timed_region(pipe, host_pool, args.steps, args.warmup, host=True, world=world, per_step=per_step)
     clocks = sampler.stop()
     scenes_total = world * BATCH * args.steps * per_step
     value = scenes_total / (ms / 1e3)

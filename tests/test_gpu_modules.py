@@ -1,5 +1,6 @@
 """-m gpu parity of the module-level drop-ins (fused inference path) against the CPU oracle (float64 conv
-stack = clean truth) and against the reference's own modules + CUDA ops (oracle/_ref) with TF32 off.
+stack = clean truth), against recorded outputs of the same modules and batches (tests/helpers.py::Recorded) and, where
+oracle/_ref is installed, against the reference's own modules + CUDA ops, with TF32 off.
 Indices bit-exact; features within 1e-3 relative (tests/helpers.py::REL_TOL)."""
 import copy
 
@@ -9,7 +10,7 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from helpers import assert_close, make_backbone, rel_err, small_sa_cfg  # noqa: E402
+from helpers import assert_close, check_backbone_vs_recorded, make_backbone, rel_err, small_sa_cfg  # noqa: E402
 from spsnet_b200 import scenes  # noqa: E402
 
 
@@ -86,54 +87,68 @@ def test_sa_module_vs_oracle(oracle, kind, n):
         np.testing.assert_array_equal(got[4].cpu().numpy().reshape(B, -1), np.asarray(want[4]).reshape(B, -1))
 
 
+def _no_tf32():
+    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
+    torch.backends.cudnn.allow_tf32 = False
+    torch.backends.cuda.matmul.allow_tf32 = False
+    return old
+
+
 @pytest.mark.parametrize("kind,n", [("l0", 4096), ("l1", 2048), ("l2", 1024), ("l3", 512)])
-def test_sa_module_vs_reference_modules(ref_ops, kind, n):
-    if ref_ops is None:
-        pytest.skip("oracle/_ref (rebuilt reference) not present")
+def test_sa_module_vs_reference_modules(ref_ops, recorded, kind, n):
+    """The drop-in module (TF32 off) against the recorded outputs of the same module and batch (tests/helpers.py::Recorded)
+    and, where oracle/_ref is installed, against the reference's own module + CUDA ops: sampled indices and new_xyz
+    bit-exact, features and class logits within 1e-3."""
     B = 2
     m, cin = _sa_module(kind, seed=1)
     m = m.cuda()
-    ref, _ = _sa_module(kind, seed=7, impl=ref_ops.modules)
-    ref = ref.cuda()
-    assert list(ref.state_dict().keys()) == list(m.state_dict().keys())
-    ref.load_state_dict(m.state_dict())
+    ref = None
+    if ref_ops is not None:
+        ref, _ = _sa_module(kind, seed=7, impl=ref_ops.modules)
+        ref = ref.cuda()
+        assert list(ref.state_dict().keys()) == list(m.state_dict().keys())
+        ref.load_state_dict(m.state_dict())
     rng = np.random.default_rng(4)
     xyz = dev(np.ascontiguousarray(scenes.make_batch(60, B, n)[:, :, :3]))
     feats = dev(rng.standard_normal((B, cin, n)).astype(np.float32))
     cls = dev(scenes.make_cls_logits(19, B, n)) if kind in ("l2", "l3") else None
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
-    torch.backends.cudnn.allow_tf32 = False
-    torch.backends.cuda.matmul.allow_tf32 = False
+    old = _no_tf32()
     try:
         with torch.no_grad():
-            want = ref(xyz, feats, cls)
             got = m(xyz, feats, cls)
-            torch.backends.cudnn.allow_tf32 = True   # the reference as shipped (cuDNN convolutions in TF32)
-            stock = ref(xyz, feats, cls)
+            if ref is not None:
+                want = ref(xyz, feats, cls)
+                torch.backends.cudnn.allow_tf32 = True   # the reference as shipped (cuDNN convolutions in TF32)
+                stock = ref(xyz, feats, cls)
     finally:
         torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
-    np.testing.assert_array_equal(got[3].cpu().numpy(), want[3].cpu().numpy())  # sampled indices, bit-exact
-    np.testing.assert_array_equal(got[0].cpu().numpy(), want[0].cpu().numpy())  # new_xyz
-    assert_close(got[1].cpu().numpy(), want[1].cpu().numpy(), what=f"{kind} new_features vs reference")
-    if want[2] is not None:
+    recorded.exact("idx", got[3])  # sampled indices, bit-exact
+    recorded.exact("new_xyz", got[0])
+    recorded.close("new_features", got[1])
+    if got[2] is not None:
         # The class logits decide the next layer's top-k picks: same 1e-3 bar as the features, no escape clause.  (The reference's
         # own stock configuration -- cuDNN TF32 -- is printed next to it: it misses the bar on some heads, the fused path, whose
         # aggregation / confidence GEMMs are fp32-grade hi + lo arithmetic, does not: scripts/diag_precision.py, six seeds,
         # profiles/r02_diag_precision.txt.)
-        e = rel_err(got[2].cpu().numpy(), want[2].cpu().numpy())
-        e_ref = rel_err(stock[2].cpu().numpy(), want[2].cpu().numpy())
-        print(f"[cls] {kind}: ours vs reference-fp32 {e:.2e}; reference stock (TF32) vs reference-fp32 {e_ref:.2e}")
-        assert e <= REL_TOL_LOGITS, f"{kind} cls vs reference: relative error {e:.3e} > {REL_TOL_LOGITS:.1e}"
+        recorded.close("cls", got[2], REL_TOL_LOGITS)
+    if ref is not None:
+        np.testing.assert_array_equal(got[3].cpu().numpy(), want[3].cpu().numpy())
+        np.testing.assert_array_equal(got[0].cpu().numpy(), want[0].cpu().numpy())
+        assert_close(got[1].cpu().numpy(), want[1].cpu().numpy(), what=f"{kind} new_features vs reference")
+        if want[2] is not None:
+            e = rel_err(got[2].cpu().numpy(), want[2].cpu().numpy())
+            e_ref = rel_err(stock[2].cpu().numpy(), want[2].cpu().numpy())
+            print(f"[cls] {kind}: ours vs reference-fp32 {e:.2e}; reference stock (TF32) vs reference-fp32 {e_ref:.2e}")
+            assert e <= REL_TOL_LOGITS, f"{kind} cls vs reference: relative error {e:.3e} > {REL_TOL_LOGITS:.1e}"
 
 
 @pytest.mark.parametrize("stype,n,npoint", [("F-FPS", 1024, 256), ("FS", 1024, 128), ("ds_FPS", 2048, 512), ("ry_FPS", 2048, 512),
                                              ("Rand", 1000, 200), ("S-FPS", 16384, 4096), ("S-FPS", 2048, 512), ("D-FPS", 3000, 777)])
-def test_every_sampler_vs_reference_modules(ref_ops, stype, n, npoint):
+def test_every_sampler_vs_reference_modules(ref_ops, recorded, stype, n, npoint):
     """Every sampler string the reference dispatches on (pointnet2_modules.py:284-419; SURVEY.md App. C) through the
-    drop-in module vs the reference module + its CUDA ops: sampled indices and new_xyz bit-exact (S-FPS incl. its
-    `< 3500 unique` fallback at the small size), features within 1e-3."""
-    if ref_ops is None:
-        pytest.skip("oracle/_ref (rebuilt reference) not present")
+    drop-in module against the recorded outputs of the same module and batch (tests/helpers.py::Recorded) and, where
+    oracle/_ref is installed, against the reference module + its CUDA ops: sampled indices and new_xyz bit-exact (S-FPS
+    incl. its `< 3500 unique` fallback at the small size), features within 1e-3."""
     from spsnet_b200 import backbone as bb
     from spsnet_b200 import pointnet2_modules as pm
 
@@ -145,29 +160,36 @@ def test_every_sampler_vs_reference_modules(ref_ops, stype, n, npoint):
     mine = pm.PointnetSAModuleMSG_WithSampling(**copy.deepcopy(kw))
     bb.randomize_bn_stats(mine, seed=3)
     mine = mine.cuda().eval()
-    ref = ref_ops.modules.PointnetSAModuleMSG_WithSampling(**copy.deepcopy(kw)).cuda().eval()
-    ref.load_state_dict(mine.state_dict())
+    ref = None
+    if ref_ops is not None:
+        ref = ref_ops.modules.PointnetSAModuleMSG_WithSampling(**copy.deepcopy(kw)).cuda().eval()
+        ref.load_state_dict(mine.state_dict())
     rng = np.random.default_rng(12)
     xyz = dev(np.ascontiguousarray(scenes.make_batch(33, B, n)[:, :, :3]))
     feats = dev(rng.standard_normal((B, cin, n)).astype(np.float32))
     stds = dev(scenes.make_stds(5, B, n)) if stype == "S-FPS" else None
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
-    torch.backends.cudnn.allow_tf32 = False
-    torch.backends.cuda.matmul.allow_tf32 = False
+    old = _no_tf32()
     try:
         with torch.no_grad():
             kws = {"stds": stds.view(B, 1, n)} if stds is not None else {}
-            torch.manual_seed(99)   # 'Rand' draws torch.randperm on the device
-            want = ref(xyz, feats, None, **kws)
+            if ref is not None:
+                torch.manual_seed(99)   # 'Rand' draws torch.randperm on the device
+                want = ref(xyz, feats, None, **kws)
             torch.manual_seed(99)
             got = mine(xyz, feats, None, **kws)
     finally:
         torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
-    np.testing.assert_array_equal(got[3].cpu().numpy(), want[3].cpu().numpy())
-    np.testing.assert_array_equal(got[0].cpu().numpy(), want[0].cpu().numpy())
-    assert_close(got[1].cpu().numpy(), want[1].cpu().numpy(), what=f"{stype} new_features vs reference")
+    recorded.exact("idx", got[3])
+    recorded.exact("new_xyz", got[0])
+    recorded.close("new_features", got[1])
     if stds is not None:
-        np.testing.assert_array_equal(got[4].cpu().numpy().reshape(B, -1), want[4].cpu().numpy().reshape(B, -1))
+        recorded.exact("stds", got[4].reshape(B, -1))
+    if ref is not None:
+        np.testing.assert_array_equal(got[3].cpu().numpy(), want[3].cpu().numpy())
+        np.testing.assert_array_equal(got[0].cpu().numpy(), want[0].cpu().numpy())
+        assert_close(got[1].cpu().numpy(), want[1].cpu().numpy(), what=f"{stype} new_features vs reference")
+        if stds is not None:
+            np.testing.assert_array_equal(got[4].cpu().numpy().reshape(B, -1), want[4].cpu().numpy().reshape(B, -1))
 
 
 def test_training_path_matches_fused(oracle):
@@ -207,25 +229,34 @@ def test_backbone_vs_oracle(oracle):
         assert_close(out["encoder_features"][2].cpu().numpy(), want["encoder_features"][2], what="layer-1 features")
 
 
-def test_backbone_vs_reference_backbone(ref_ops):
-    """Full SA stack against the UNMODIFIED reference backbone + modules + CUDA ops on the same GPU.
+def test_backbone_vs_reference_backbone(ref_ops, recorded):
+    """Full SA stack (TF32 off) against a recorded forward of the same weights and batch
+    (tests/helpers.py::check_backbone_vs_recorded) and, where oracle/_ref is installed, against the UNMODIFIED reference
+    backbone + modules + CUDA ops on the same GPU.
 
-    The two D-FPS layers are compared end to end (bit-exact).  From the first score-based layer on, the
-    sampled ORDER depends on the last bits of the confidence logits (cuDNN vs our GEMM summation order), so
-    an end-to-end index comparison is ill-posed for ANY fp32 implementation; every layer is therefore also
-    checked teacher-forced: our module gets exactly the tensors the reference module received and must
-    return bit-identical sample indices / new_xyz and features within 1e-3."""
+    Against the reference the two D-FPS layers are compared end to end (bit-exact).  From the first score-based layer on, the
+    sampled ORDER depends on the last bits of the confidence logits (cuDNN vs our GEMM summation order), so an end-to-end
+    index comparison is ill-posed for ANY fp32 implementation; every layer is therefore also checked teacher-forced: our
+    module gets exactly the tensors the reference module received and must return bit-identical sample indices / new_xyz
+    and features within 1e-3."""
+    net = make_backbone(small_sa_cfg((1024, 256, 128, 64)), seed=4).cuda()
+    B, N = 2, 4096
+    pts = dev(scenes.to_points(scenes.make_batch(90, B, N)))
+    old = _no_tf32()
+    try:
+        with torch.no_grad():
+            got = net({"batch_size": B, "points": pts.clone()})
+    finally:
+        torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
+    check_backbone_vs_recorded(recorded, got)
     if ref_ops is None:
-        pytest.skip("oracle/_ref (rebuilt reference) not present")
+        return
     import importlib
 
     ref_bb = importlib.import_module("pcdet.models.backbones_3d.IASSD_backbone")
-    net = make_backbone(small_sa_cfg((1024, 256, 128, 64)), seed=4).cuda()
     ref = ref_bb.IASSD_Backbone(small_sa_cfg((1024, 256, 128, 64)), num_class=3, input_channels=4).cuda().eval()
     assert list(ref.state_dict().keys()) == list(net.state_dict().keys())
     ref.load_state_dict(net.state_dict())
-    B, N = 2, 4096
-    pts = dev(scenes.to_points(scenes.make_batch(90, B, N)))
     captured = {}
 
     def mk_hook(i):
@@ -234,13 +265,10 @@ def test_backbone_vs_reference_backbone(ref_ops):
         return hook
 
     hooks = [m.register_forward_hook(mk_hook(i), with_kwargs=True) for i, m in enumerate(ref.SA_modules)]
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
-    torch.backends.cudnn.allow_tf32 = False
-    torch.backends.cuda.matmul.allow_tf32 = False
+    old = _no_tf32()
     try:
         with torch.no_grad():
             want = ref({"batch_size": B, "points": pts.clone()})
-            got = net({"batch_size": B, "points": pts.clone()})
             for i in (1, 2):  # D-FPS layers: exact end to end
                 np.testing.assert_array_equal(got["encoder_xyz"][i].cpu().numpy(), want["encoder_xyz"][i].cpu().numpy(),
                                               err_msg=f"encoder_xyz[{i}] (D-FPS sampling) differs from the reference")
@@ -268,11 +296,10 @@ def test_backbone_vs_reference_backbone(ref_ops):
             h.remove()
 
 
-def test_stability_generator_vs_reference(ref_ops):
-    """SPSNet stability generator (eval branch): stds = sum exp(0.5 * fc2(SA(points))) against the reference's own
+def test_stability_generator_vs_reference(ref_ops, recorded):
+    """SPSNet stability generator (eval branch): stds = sum exp(0.5 * fc2(SA(points))) against the recorded outputs of the
+    same weights and points (tests/helpers.py::Recorded) and, where oracle/_ref is installed, against the reference's own
     PointnetSampling module + CUDA ops with the same weights (identity sampling: every point is a centre)."""
-    if ref_ops is None:
-        pytest.skip("oracle/_ref (rebuilt reference) not present")
     from spsnet_b200 import backbone as bb
     from spsnet_b200 import stability as st
 
@@ -283,35 +310,42 @@ def test_stability_generator_vs_reference(ref_ops):
     gen = st.Generate_center(cfg)
     bb.randomize_bn_stats(gen, seed=5)
     gen = gen.cuda().eval()
-    sa = cfg["SA_CONFIG"]
-    ref_sa = ref_ops.modules.PointnetSampling(
-        npoint_list=sa["NPOINT_LIST"][0], sample_range_list=sa["SAMPLE_RANGE_LIST"][0], sample_type_list=sa["SAMPLE_METHOD_LIST"][0],
-        radii=sa["RADIUS_LIST"][0], nsamples=sa["NSAMPLE_LIST"][0], mlps=[[1] + list(m) for m in sa["MLPS"][0]], use_xyz=True,
-        dilated_group=False, aggregation_mlp=list(sa["AGGREGATION_MLPS"][0])).cuda().eval()
-    mine = gen.feature_extract.SA_modules[0]
-    assert list(ref_sa.state_dict().keys()) == list(mine.state_dict().keys())
-    ref_sa.load_state_dict(mine.state_dict())
     pts = scenes.make_batch(70, B, N)
     points = dev(scenes.to_points(pts))
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
-    torch.backends.cudnn.allow_tf32 = False
-    torch.backends.cuda.matmul.allow_tf32 = False
+    old = _no_tf32()
     try:
         with torch.no_grad():
             out = gen({"batch_size": B, "points": points.clone()})
-            xyz = dev(np.ascontiguousarray(pts[:, :, :3]))
-            feats = dev(np.ascontiguousarray(pts[:, :, 3:].transpose(0, 2, 1)))
-            r_xyz, r_feat, r_idx = ref_sa(xyz, feats, None)
-            logvar = gen.feature_encoder.fc2(r_feat.permute(0, 2, 1).contiguous())
-            want = torch.sum(torch.exp(0.5 * logvar), dim=-1)
     finally:
         torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
     assert out["stds"].shape == (B, N)
-    np.testing.assert_array_equal(out["encoder_xyz"][1].cpu().numpy(), r_xyz.cpu().numpy())
-    assert_close(out["soc_feature"].cpu().numpy(), r_feat.permute(0, 2, 1).cpu().numpy(), what="generator soc_feature")
-    e = rel_err(out["stds"].cpu().numpy(), want.cpu().numpy())
-    print(f"[stability] stds rel err vs reference composition {e:.2e}")
-    assert e <= 1e-3
+    recorded.exact("encoder_xyz1", out["encoder_xyz"][1])
+    recorded.close("soc_feature", out["soc_feature"])
+    recorded.close("stds", out["stds"])
+    if ref_ops is not None:
+        sa = cfg["SA_CONFIG"]
+        ref_sa = ref_ops.modules.PointnetSampling(
+            npoint_list=sa["NPOINT_LIST"][0], sample_range_list=sa["SAMPLE_RANGE_LIST"][0], sample_type_list=sa["SAMPLE_METHOD_LIST"][0],
+            radii=sa["RADIUS_LIST"][0], nsamples=sa["NSAMPLE_LIST"][0], mlps=[[1] + list(m) for m in sa["MLPS"][0]], use_xyz=True,
+            dilated_group=False, aggregation_mlp=list(sa["AGGREGATION_MLPS"][0])).cuda().eval()
+        mine = gen.feature_extract.SA_modules[0]
+        assert list(ref_sa.state_dict().keys()) == list(mine.state_dict().keys())
+        ref_sa.load_state_dict(mine.state_dict())
+        old = _no_tf32()
+        try:
+            with torch.no_grad():
+                xyz = dev(np.ascontiguousarray(pts[:, :, :3]))
+                feats = dev(np.ascontiguousarray(pts[:, :, 3:].transpose(0, 2, 1)))
+                r_xyz, r_feat, r_idx = ref_sa(xyz, feats, None)
+                logvar = gen.feature_encoder.fc2(r_feat.permute(0, 2, 1).contiguous())
+                want = torch.sum(torch.exp(0.5 * logvar), dim=-1)
+        finally:
+            torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
+        np.testing.assert_array_equal(out["encoder_xyz"][1].cpu().numpy(), r_xyz.cpu().numpy())
+        assert_close(out["soc_feature"].cpu().numpy(), r_feat.permute(0, 2, 1).cpu().numpy(), what="generator soc_feature")
+        e = rel_err(out["stds"].cpu().numpy(), want.cpu().numpy())
+        print(f"[stability] stds rel err vs reference composition {e:.2e}")
+        assert e <= 1e-3
     # the stds drive SPSNet-IA's stability-aware sampling end to end
     net = make_backbone(small_sa_cfg((512, 128, 64, 32)), seed=2, cls=bb.PAGNet_Backbone)
     net.model_cfg.SA_CONFIG["SAMPLE_METHOD_LIST"][2] = ["sss_aware"]

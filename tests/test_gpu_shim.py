@@ -18,6 +18,8 @@ from spsnet_b200 import configs, scenes  # noqa: E402
 
 
 def test_reference_python_layer_runs_unmodified_over_the_shim(ref_ops, ref_det, tmp_path):
+    if ref_ops is None or ref_det is None:
+        pytest.skip("runs the reference's own Python layer from oracle/_ref (oracle/build_ref.sh), which the repository does not hold")
     out = tmp_path / "shim.npz"
     r = subprocess.run([sys.executable, str(ROOT / "tests" / "run_reference_over_shim.py"), str(out)], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]

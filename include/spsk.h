@@ -144,8 +144,11 @@ SPSK_API int spsk_scatter_grad(int b, int c, int n, long long l_per_scene, int c
  * score = sigmoid(max_c cls) * (1 - sigmoid(stds/8 - 3)) (pointnet2_modules.py:293-303).
  * cls (b,n,num_class) f32; stds (b,n) f32 or NULL; idx (b,npoint) out, ordered by descending score,
  * ties broken by ascending point index; scores (b,npoint) out or NULL (the picked scores).
- * n <= SPSK_TOPK_MAX_N. */
-#define SPSK_TOPK_MAX_N 16384
+ * n <= SPSK_TOPK_MAX_N, in one launch and without workspace: n <= 16384 sorts each scene in one CTA's shared
+ * memory; 16384 < n <= 262144 sorts it across a thread-block cluster of ceil_pow2(n) / 16384 CTAs (2, 4, 8 or
+ * 16; 128 KB of shared memory each).  A 16-CTA cluster (n > 131072) is a non-portable size: a device that
+ * cannot schedule one returns SPSK_ERR_UNSUPPORTED. */
+#define SPSK_TOPK_MAX_N 262144
 SPSK_API int spsk_score_topk(int b, int n, int num_class, int npoint, const float *cls, const float *stds,
                     int *idx, float *scores, spsk_stream_t stream);
 

@@ -84,4 +84,18 @@ __device__ __forceinline__ uint32_t fps_rank(uint32_t k, uint32_t s_mask, uint32
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }
 
+// ---- thread-block clusters (fps.cu, topk.cu) ------------------------------------------------------
+__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
+__device__ __forceinline__ uint32_t cluster_nctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r)); return r; }
+__device__ __forceinline__ void cluster_sync_all() {
+    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// the shared::cluster address of the variable at shared::cta address `local_addr` in CTA `cta` of this cluster
+__device__ __forceinline__ uint32_t cluster_map_shared(uint32_t local_addr, uint32_t cta) {
+    uint32_t r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(cta));
+    return r;
+}
+
 }  // namespace spsk

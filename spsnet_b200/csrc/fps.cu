@@ -157,20 +157,12 @@ fps_kernel_1024(int n, int m, const float *__restrict__ src, float *__restrict__
 // store itself completes transaction bytes on the receiver's mbarrier, so there is no cluster barrier and no fence on the
 // chain -- and every warp picks the winner among the csize records.  The winner's coordinates travel with the record, so
 // no CTA ever reads another CTA's points.
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ uint32_t cluster_nctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 // st.async: the store itself completes `16` transaction bytes on the consumer CTA's mbarrier -- data and signal in one
 // message, no fence and no cluster barrier on the per-iteration chain (measured: barrier.cluster arrive.release +
 // wait.acquire costs 518 cycles at 4 x 512 threads and compiles to MEMBAR.ALL.GPU + CCTL.IVALL around it).
 __device__ __forceinline__ void st_async_v4(const void *local_rec, const void *local_bar, uint32_t cta, uint4 v) {
-    const uint32_t la = (uint32_t)__cvta_generic_to_shared(local_rec), lb = (uint32_t)__cvta_generic_to_shared(local_bar);
-    uint32_t ra, rb;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(la), "r"(cta));
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rb) : "r"(lb), "r"(cta));
+    const uint32_t ra = cluster_map_shared((uint32_t)__cvta_generic_to_shared(local_rec), cta);
+    const uint32_t rb = cluster_map_shared((uint32_t)__cvta_generic_to_shared(local_bar), cta);
     asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];"
                  ::"r"(ra), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "r"(rb) : "memory");
 }
@@ -190,9 +182,7 @@ __device__ __forceinline__ void xbar_wait(uint64_t *bar, uint32_t parity) {
     }
 }
 __device__ __forceinline__ void st_cluster_v4(const void *local_ptr, uint32_t cta, uint4 v) {
-    const uint32_t la = (uint32_t)__cvta_generic_to_shared(local_ptr);
-    uint32_t ra;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(la), "r"(cta));
+    const uint32_t ra = cluster_map_shared((uint32_t)__cvta_generic_to_shared(local_ptr), cta);
     asm volatile("st.shared::cluster.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(ra), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
 

@@ -368,7 +368,8 @@ class GroupAll(nn.Module):
 def score_topk(cls_features: torch.Tensor, npoint: int, stds: torch.Tensor | None = None,
                return_scores: bool = False):
     """ctr/cls-aware (reference pointnet2_modules.py:287-291) or, with `stds`, SPSNet stability-aware
-    (:293-303) down-sampling indices: (B, npoint) int32, descending score, ties by ascending index."""
+    (:293-303) down-sampling indices: (B, npoint) int32, descending score, ties by ascending index.  One kernel launch
+    for N up to 262144 (one CTA per scene up to 16384 points, a thread-block cluster of up to 16 CTAs above)."""
     _chk(cls_features, "cls_features", torch.float32, 3)
     B, N, nc = cls_features.shape
     if stds is not None:

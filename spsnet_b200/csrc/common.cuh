@@ -38,12 +38,18 @@ constexpr float FP16_MAX = 65504.f;
 
 static inline cudaStream_t as_stream(spsk_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
 
+// index of the current device into the per-device tables below
+static inline int device_slot() {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
+    return dev;
+}
+
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-device attribute: set it once per (kernel, device).
 struct SmemAttrOnce {
     bool done[64] = {};
     int ensure(const void *func, int bytes, const char *what) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
+        const int dev = device_slot();
         if (done[dev]) return 0;
         cudaError_t e = cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
         if (e != cudaSuccess) return cuda_fail(e, what);
@@ -81,6 +87,12 @@ __device__ __forceinline__ float sqdist3(float ax, float ay, float az, float bx,
 __device__ __forceinline__ uint32_t fps_rank(uint32_t k, uint32_t s_mask, uint32_t s_log2) {
     return __brev(k & s_mask) | (k >> s_log2);
 }
+// The inverse of fps_rank: the point index k whose rank is `rank`.  s_log2 == 0 (S = 1) keeps every bit of the rank; the
+// general mask would shift by 32, which is undefined.
+__device__ __forceinline__ uint32_t fps_unrank(uint32_t rank, uint32_t s_mask, uint32_t s_log2) {
+    const uint32_t low_mask = s_log2 ? ((1u << (32u - s_log2)) - 1u) : 0xFFFFFFFFu;
+    return (__brev(rank) & s_mask) | ((rank & low_mask) << s_log2);
+}
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }
 
@@ -96,6 +108,54 @@ __device__ __forceinline__ uint32_t cluster_map_shared(uint32_t local_addr, uint
     uint32_t r;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(cta));
     return r;
+}
+
+// What launch_cluster has set up or learned for one kernel, per device.  Each cluster kernel owns one, as a static beside
+// its launch: two kernels of the same function type (e.g. a kernel with and without its profiling counters) must not share
+// it, or the second would never get its shared-memory attribute.
+struct ClusterKernelState {
+    SmemAttrOnce smem;
+    signed char schedulable[64] = {};   // csize > 8: 0 = not asked yet, 1 = yes, -1 = no
+};
+// launch_cluster's result when the device cannot co-schedule a cluster of that size of that kernel.  It is no CUDA error
+// and sets no message: each caller decides what to do instead.  Distinct from SPSK_OK and every SPSK_ERR_* code.
+constexpr int SPSK_CLUSTER_UNSCHEDULABLE = 1;
+
+// Launches `kern` on nclusters clusters of csize CTAs (along x) with `smem` bytes of dynamic shared memory each.  Clusters of
+// more than 8 CTAs are a non-portable size: the kernel opts in and the device is asked once whether it can co-schedule one.
+// The answer cannot change for a (kernel, device, cluster shape), and both callers use a single size above 8 (16), so it is
+// cached per (kernel, device) and never asked again, e.g. inside a CUDA-graph capture.
+template <typename... KArgs, typename... Args>
+static int launch_cluster(ClusterKernelState &state, void (*kern)(KArgs...), const char *name, int nclusters, int csize,
+                          int threads, size_t smem, cudaStream_t st, Args... args) {
+    if (int rc = state.smem.ensure(reinterpret_cast<const void *>(kern), (int)smem, name)) return rc;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(nclusters * csize));
+    cfg.blockDim = dim3((unsigned)threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = (unsigned)csize;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    if (csize > 8) {
+        signed char &ok = state.schedulable[device_slot()];
+        if (ok == 0) {
+            int clusters = 0;
+            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+            if (e == cudaSuccess) e = cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg);
+            if (e != cudaSuccess) (void)cudaGetLastError();
+            ok = e == cudaSuccess && clusters >= 1 ? 1 : -1;
+        }
+        if (ok < 0) return SPSK_CLUSTER_UNSCHEDULABLE;
+    }
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args...);
+    if (e != cudaSuccess) return cuda_fail(e, name);
+    SPSK_LAUNCH_CHECK(name);
+    return SPSK_OK;
 }
 
 }  // namespace spsk

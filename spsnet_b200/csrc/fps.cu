@@ -2,18 +2,16 @@
 //
 // Replaces farthest_point_sampling_kernel / furthest_point_sampling_with_dist_kernel of the
 // reference (src/sampling_gpu.cu:93-209, 256-371).  Same arithmetic, same winners (bit-exact,
-// including the block-tree tie-break, see common.cuh::fps_rank), different machine mapping:
+// including the block-tree tie-break, see common.cuh::fps_rank), different machine mapping.
+// FPS is latency bound: m-1 strictly sequential arg-max steps per scene.
 //
-//   reference                                     here
-//   -----------------------------------------     ------------------------------------------------
-//   running minima `temp` in global memory,       running minima in REGISTERS (P per thread), xyz
-//   xyz re-read from global every iteration       staged once into shared memory (SoA) and, for
-//                                                 P <= 8, also held in registers
-//   11 __syncthreads per iteration (smem tree)    1 __syncthreads per iteration: REDUX.MAX warp
-//                                                 arg-max -> one smem slot per warp (double
-//                                                 buffered) -> REDUX.MAX again in every warp
-//
-// FPS is latency bound: m-1 strictly sequential arg-max steps per scene.  One CTA per scene.
+//   D-FPS, 1024 <= n <= 16384        fps_pruned_kernel, one CTA per scene: only the sub-buckets of Morton-sorted points that
+//                                    a new sample can change are updated; running minima in tensor or shared memory
+//   D-FPS, 16384 < n <= 262144       fps_pruned_kernel on one 2/4/8/16-CTA cluster per scene, arg-max across the cluster
+//                                    through distributed shared memory
+//   n < 1024, F-FPS, SPSK_FPS=dense  fps_kernel_1024 / fps_kernel: every point every step, running minima in registers, xyz
+//                                    staged once into shared memory, 1 __syncthreads per step (the reference takes 11)
+//   larger scenes                    fps_generic_kernel: running minima in the caller's `temp`
 #include "mma_ptx.cuh"
 #include <stdlib.h>
 
@@ -41,10 +39,7 @@ __device__ __forceinline__ uint32_t block_argmax(uint32_t u, uint32_t inv_rank, 
     const uint32_t m2 = __reduce_max_sync(0xFFFFFFFFu, v.x);
     const uint32_t c2 = (v.x == m2) ? v.y : 0u;
     const uint32_t r2 = __reduce_max_sync(0xFFFFFFFFu, c2);
-    // invert rank(k) = brev(k & s_mask) | (k >> s_log2)
-    const uint32_t rank = ~r2;
-    const uint32_t low_mask = s_log2 ? ((1u << (32u - s_log2)) - 1u) : 0xFFFFFFFFu;
-    return (__brev(rank) & s_mask) | ((rank & low_mask) << s_log2);
+    return fps_unrank(~r2, s_mask, s_log2);
 }
 
 // Main kernel, n >= 1024 (reference block size S = 1024 = T).  All points of one thread (k = tid + p*T)
@@ -137,7 +132,7 @@ fps_kernel_1024(int n, int m, const float *__restrict__ src, float *__restrict__
 // Spatially pruned D-FPS (same winners, far less work per step).
 //
 // The update temp[k] = min(temp[k], |p_k - q|^2) cannot change temp[k] when |p_k - q|^2 >= temp[k].  Points
-// are sorted once along a Morton curve (in-kernel bitonic sort of 32-bit (cell code, index) keys) and cut
+// are sorted once along a Morton curve (in-kernel counting sort by cell code) and cut
 // into sub-buckets of 32 consecutive points (one per lane).  Each sub-bucket keeps its bounding box, the
 // maximum of its running minima (bmax) and the rank of its best point.  Per step a lane evaluates the
 // box-to-query lower bound lb of "its" sub-bucket with THE SAME fp32 expression as the distance itself
@@ -148,8 +143,9 @@ fps_kernel_1024(int n, int m, const float *__restrict__ src, float *__restrict__
 // a handful of the 512 sub-buckets).  The sort only decides HOW MUCH is skipped, never the result.
 //
 // 512 threads, P points per lane (P*512 >= n), sub-bucket s = p*16 + warp (round-robin over warps so that
-// neighbouring sub-buckets are processed by different warps), sorted xyz in shared memory (SoA), running
-// minima / original indices in registers, orig->sorted position map (u16) in shared memory.
+// neighbouring sub-buckets are processed by different warps), sorted xyz in shared memory (SoA), original
+// indices in registers, running minima in tensor or shared memory (see below), orig->sorted position map (u16)
+// in shared memory.
 // CL = true: a thread-block CLUSTER per scene (n > 16384, e.g. Waymo's 65536 points): CTA r of the cluster owns the
 // contiguous index range [r*chunk, (r+1)*chunk), prunes and updates it exactly like the single-CTA kernel, and the
 // per-iteration arg-max is completed across the cluster through distributed shared memory: each CTA reduces its 16 warp
@@ -166,12 +162,7 @@ __device__ __forceinline__ void st_async_v4(const void *local_rec, const void *l
     asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];"
                  ::"r"(ra), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "r"(rb) : "memory");
 }
-__device__ __forceinline__ void xbar_init(uint64_t *bar) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)) : "memory");
-}
-__device__ __forceinline__ void xbar_arm(uint64_t *bar, uint32_t bytes) {   // the one local arrival + the bytes this phase will receive
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(bytes) : "memory");
-}
+// Not mma_ptx.cuh's mbar_wait: its spin counter and trap would add instructions to the per-step chain.
 __device__ __forceinline__ void xbar_wait(uint64_t *bar, uint32_t parity) {
     const uint32_t a = (uint32_t)__cvta_generic_to_shared(bar);
     uint32_t done = 0;
@@ -181,40 +172,35 @@ __device__ __forceinline__ void xbar_wait(uint64_t *bar, uint32_t parity) {
                      : "=r"(done) : "r"(a), "r"(parity) : "memory");
     }
 }
-__device__ __forceinline__ void st_cluster_v4(const void *local_ptr, uint32_t cta, uint4 v) {
-    const uint32_t ra = cluster_map_shared((uint32_t)__cvta_generic_to_shared(local_ptr), cta);
-    asm volatile("st.shared::cluster.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(ra), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
 
 // PROF: compile the phase counters in (spsk_fps_set_profile).  They are predicated instructions, but on this latency chain
 // every issue slot counts: 16 warps x ~40 predicated-off instructions per iteration were ~10 % of the iteration.
 //
-// TM: the running minima (and each point's tie-break key ~rank) live in TENSOR MEMORY instead of registers.  The minima of a
-// lane are private to it, which is exactly the access pattern tcgen05.ld/st offer (a warp reaches the 32 TMEM lanes of its
-// quarter; column = sub-bucket), and -- unlike registers -- the column index is DYNAMIC: a visited sub-bucket is one generic
-// loop body (ffs over the ballot mask, 12-cycle TMEM load, distance, TMEM store, two REDUX) instead of a 32-case ladder of
-// warp-uniform branches around 32 statically indexed copies of the body.  Measured with the phase counters (round 2): the
-// ladder + its reconvergence points cost ~400-500 cycles per visited sub-bucket on the critical warp of an iteration; the
-// generic body ~160.  Shared memory cannot take the minima (xyz 192 KB + index map 32 KB already fill it at 16384 points);
-// the 256 KB of TMEM are otherwise unused by this kernel.  Layout: warp w owns columns [(w / 4) * 2P, +2P) of lane quarter
-// w % 4; sub-bucket p = columns (2p, 2p + 1) = (running minimum bits, ~rank or 0 for padding).
-// ST (storage of the running minima): 0 = registers + ladder (the round-1 kernel), 1 = tensor memory (TM above), 2 = shared
-// memory (small scenes, P <= 8: the minima fit next to xyz, and a small CTA must not hold TMEM columns -- it shares its SM with
-// sa_mma CTAs that allocate all 512).  1 and 2 run the same generic visit loop.
-template <int P, bool CL, int LADDER, bool PROF, int ST>
+// Running minima (and each point's tie-break key ~rank): the index of a visited sub-bucket is DYNAMIC, so a visit is one
+// generic loop body (ffs over the ballot mask, load, distance, store, two REDUX).  In registers the index would have to be
+// static: the round-1 kernel ran a 32-case ladder of warp-uniform branches around 32 statically indexed copies of the body,
+// ~400-500 cycles per visited sub-bucket on the critical warp against ~160 for the generic body (phase counters, round 2).
+//  - P >= 16 (more than 4096 points per CTA, and every cluster CTA): TENSOR MEMORY.  The minima of a lane are private to it,
+//    which is exactly the access pattern tcgen05.ld/st offer (a warp reaches the 32 TMEM lanes of its quarter; column =
+//    sub-bucket; 12-cycle load).  Shared memory cannot take them (xyz 192 KB + index map 32 KB already fill it at 16384
+//    points); the 256 KB of TMEM are otherwise unused by this kernel.  Layout: warp w owns columns [(w / 4) * 2P, +2P) of lane
+//    quarter w % 4; sub-bucket p = columns (2p, 2p + 1) = (running minimum bits, ~rank or 0 for padding).
+//  - P <= 8: SHARED memory, next to xyz.  Such a small CTA must not hold TMEM columns: it shares its SM with sa_mma CTAs that
+//    allocate all 512.
+template <int P, bool CL, bool PROF>
 __global__ void __launch_bounds__(512, 1)
 fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__restrict__ temp, int *__restrict__ idx,
-                  unsigned long long *__restrict__ prof, int bitonic) {
+                  unsigned long long *__restrict__ prof) {
     constexpr int T = 512, W = 16, NP = T * P;
-    constexpr bool TM = ST == 1, SM = ST == 2, GEN = ST != 0;
+    constexpr bool TM = P >= 16;
+    static_assert(TM || !CL, "the shared-memory minima follow the index map, which only a single-CTA scene has");
     constexpr uint32_t s_mask = 1023u, s_log2 = 10u;   // reference block size is 1024 for n >= 1024
     extern __shared__ float smem[];
     __shared__ float red[6][W];
     float *sx = smem, *sy = smem + NP, *sz = smem + 2 * NP;
-    uint32_t *keys = reinterpret_cast<uint32_t *>(smem);              // sort phase only (aliases sx)
     unsigned short *pos_of = reinterpret_cast<unsigned short *>(smem + 3 * NP);
-    float *stmp = smem + 3 * NP + (CL ? 0 : NP / 2);                   // ST == 2: running minima by sorted position ...
-    uint32_t *sir = reinterpret_cast<uint32_t *>(stmp + NP);          // ... and ~rank (0 = padding)
+    float *stmp = smem + 3 * NP + NP / 2;                        // !TM: running minima by sorted position ...
+    uint32_t *sir = reinterpret_cast<uint32_t *>(stmp + NP);    // ... and ~rank (0 = padding)
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t crank = CL ? cluster_ctarank() : 0u, csize = CL ? cluster_nctarank() : 1u;
     const size_t scene = CL ? blockIdx.x / csize : blockIdx.x;
@@ -262,7 +248,7 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
     // order: a counting sort by the top log2(NP) bits of the (7+7-bit xy Morton, 4-bit z) cell code -- as many cells as point
     // slots -- replaces the full bitonic sort of (code, index) keys, which cost ~8 % of the 16384 -> 4096 kernel (105 passes over
     // 16384 keys, a block barrier each).  Shared-memory atomics, one scan, one scatter; the order inside a cell is whatever the
-    // atomics give (run to run the sub-buckets may differ, the samples cannot).  `bitonic` keeps the round-1 sort for A/B.
+    // atomics give (run to run the sub-buckets may differ, the samples cannot).
     auto cell_code = [&](int i) -> uint32_t {
         const float x = __ldg(base + (size_t)i * 3), y = __ldg(base + (size_t)i * 3 + 1), z = __ldg(base + (size_t)i * 3 + 2);
         uint32_t cx = min(127, max(0, (int)((x - org[0]) * scl[0])));
@@ -272,81 +258,50 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
         cy = (cy | (cy << 4)) & 0x0F0Fu; cy = (cy | (cy << 2)) & 0x3333u; cy = (cy | (cy << 1)) & 0x5555u;
         return (((cx | (cy << 1)) & 0x3FFFu) << 4) | cz;   // 18 bits
     };
-    unsigned short *sorted16 = reinterpret_cast<unsigned short *>(smem) + 3 * NP;   // counting sort: point index by sorted position
-    if (bitonic) {
-        // keys: cell code << 14 | index ; padding sorts last
-        for (int i = tid; i < NP; i += T) {
-            uint32_t key = 0xFFFFFFFFu;
-            // the top cell's last z slice is merged into its neighbour so that no real key equals the padding key 0xFFFFFFFF
-            // (code 0x3FFFF with local index 16383 would)
-            if (i < n) key = (min(cell_code(i), 0x3FFFEu) << 14) | (uint32_t)i;
-            keys[i] = key;
-        }
-        __syncthreads();
-        for (int k = 2; k <= NP; k <<= 1) {
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int i = tid; i < NP; i += T) {
-                    const int ixj = i ^ j;
-                    if (ixj > i) {
-                        const uint32_t a = keys[i], b = keys[ixj];
-                        const bool up = (i & k) == 0;
-                        if (up ? (a > b) : (a < b)) { keys[i] = b; keys[ixj] = a; }
-                    }
-                }
-                __syncthreads();
-            }
-        }
-    } else {
-        // [hist u32 x NP][codes u16 x NP][sorted u16 x NP] = 8 NP bytes of the 12 NP-byte xyz region
-        uint32_t *hist = reinterpret_cast<uint32_t *>(smem);
-        unsigned short *codes = reinterpret_cast<unsigned short *>(smem) + 2 * NP;
-        constexpr int CB = (P == 2 ? 10 : P == 4 ? 11 : P == 8 ? 12 : P == 16 ? 13 : 14);   // log2(NP) cells
-        for (int i = tid; i < NP; i += T) { hist[i] = 0u; sorted16[i] = 0xFFFFu; }
-        __syncthreads();
-        for (int i = tid; i < n; i += T) {
-            const uint32_t c = cell_code(i) >> (18 - CB);
-            codes[i] = (unsigned short)c;
-            atomicAdd(&hist[c], 1u);
-        }
-        __syncthreads();
-        // exclusive scan over the NP counters: thread t owns counters [t P, (t + 1) P)
-        uint32_t loc[P], run = 0u;
-#pragma unroll
-        for (int p = 0; p < P; ++p) { loc[p] = run; run += hist[tid * P + p]; }
-        uint32_t inc = run;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t up = __shfl_up_sync(0xFFFFFFFFu, inc, o);
-            if (lane >= o) inc += up;
-        }
-        uint32_t *wsum = reinterpret_cast<uint32_t *>(&red[0][0]);   // 16 warp totals (red is free again: the box is reduced)
-        __syncthreads();
-        if (lane == 31) wsum[warp] = inc;
-        __syncthreads();
-        uint32_t wbase = 0u;
-        for (int w = 0; w < warp; ++w) wbase += wsum[w];
-        const uint32_t excl = wbase + inc - run;
-#pragma unroll
-        for (int p = 0; p < P; ++p) hist[tid * P + p] = excl + loc[p];
-        __syncthreads();
-        for (int i = tid; i < n; i += T) sorted16[atomicAdd(&hist[codes[i]], 1u)] = (unsigned short)i;
-        __syncthreads();
+    // [hist u32 x NP][codes u16 x NP][sorted u16 x NP] = 8 NP bytes of the 12 NP-byte xyz region
+    uint32_t *hist = reinterpret_cast<uint32_t *>(smem);
+    unsigned short *codes = reinterpret_cast<unsigned short *>(smem) + 2 * NP;
+    unsigned short *sorted16 = reinterpret_cast<unsigned short *>(smem) + 3 * NP;   // point index by sorted position
+    constexpr int CB = (P == 2 ? 10 : P == 4 ? 11 : P == 8 ? 12 : P == 16 ? 13 : 14);   // log2(NP) cells
+    for (int i = tid; i < NP; i += T) { hist[i] = 0u; sorted16[i] = 0xFFFFu; }
+    __syncthreads();
+    for (int i = tid; i < n; i += T) {
+        const uint32_t c = cell_code(i) >> (18 - CB);
+        codes[i] = (unsigned short)c;
+        atomicAdd(&hist[c], 1u);
     }
+    __syncthreads();
+    // exclusive scan over the NP counters: thread t owns counters [t P, (t + 1) P)
+    uint32_t loc[P], run = 0u;
+#pragma unroll
+    for (int p = 0; p < P; ++p) { loc[p] = run; run += hist[tid * P + p]; }
+    uint32_t inc = run;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t up = __shfl_up_sync(0xFFFFFFFFu, inc, o);
+        if (lane >= o) inc += up;
+    }
+    uint32_t *wsum = reinterpret_cast<uint32_t *>(&red[0][0]);   // 16 warp totals (red is free again: the box is reduced)
+    __syncthreads();
+    if (lane == 31) wsum[warp] = inc;
+    __syncthreads();
+    uint32_t wbase = 0u;
+    for (int w = 0; w < warp; ++w) wbase += wsum[w];
+    const uint32_t excl = wbase + inc - run;
+#pragma unroll
+    for (int p = 0; p < P; ++p) hist[tid * P + p] = excl + loc[p];
+    __syncthreads();
+    for (int i = tid; i < n; i += T) sorted16[atomicAdd(&hist[codes[i]], 1u)] = (unsigned short)i;
+    __syncthreads();
     // ---- take ownership: slot p of this lane = sorted position ((p*W + warp)*32 + lane)
     uint32_t oidx[P];
-    float tmp[GEN ? 1 : P];
 #pragma unroll
     for (int p = 0; p < P; ++p) {
-        const int spos = (p * W + warp) * 32 + lane;
-        if (bitonic) {
-            oidx[p] = keys[spos];
-        } else {
-            const uint32_t v = sorted16[spos];
-            oidx[p] = v == 0xFFFFu ? 0xFFFFFFFFu : v;
-        }
+        const uint32_t v = sorted16[(p * W + warp) * 32 + lane];
+        oidx[p] = v == 0xFFFFu ? 0xFFFFFFFFu : v;
     }
     if (TM) tc_fence_before();
-    __syncthreads();   // keys consumed; the region becomes sx/sy/sz
+    __syncthreads();   // sorted16 consumed; the region becomes sx/sy/sz
     uint32_t tbase = 0u;   // TM: this warp's first column in its lane quarter
     if (TM) {
         tc_fence_after();
@@ -356,15 +311,14 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
     for (int p = 0; p < P; ++p) {
         const int pos = (p * W + warp) * 32 + lane;
         const bool valid = oidx[p] != 0xFFFFFFFFu;
-        const uint32_t oi = valid ? (oidx[p] & 0x3FFFu) : 0u;   // index inside the owned range
+        const uint32_t oi = valid ? oidx[p] : 0u;                // index inside the owned range
         oidx[p] = valid ? oi + (uint32_t)gbase : 0xFFFFFFFFu;   // index inside the scene (decides the tie-break rank)
         sx[pos] = valid ? __ldg(base + (size_t)oi * 3) : 0.f;
         sy[pos] = valid ? __ldg(base + (size_t)oi * 3 + 1) : 0.f;
         sz[pos] = valid ? __ldg(base + (size_t)oi * 3 + 2) : 0.f;
         const float t0 = valid ? (temp ? temp[oidx[p]] : 1e10f) : -1.f;
         if (TM) tmem_st_x2(tbase + 2u * p, __float_as_uint(t0), valid ? ~fps_rank(oidx[p], s_mask, s_log2) : 0u);
-        else if (SM) { stmp[pos] = t0; sir[pos] = valid ? ~fps_rank(oidx[p], s_mask, s_log2) : 0u; }
-        else tmp[p] = t0;
+        else { stmp[pos] = t0; sir[pos] = valid ? ~fps_rank(oidx[p], s_mask, s_log2) : 0u; }
         if (!CL && valid) pos_of[oi] = (unsigned short)pos;
     }
     if (TM) tmem_wait_st();
@@ -394,9 +348,9 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
 
     // Per iteration (the m-1 iterations are strictly sequential, so this loop is a latency chain):
     //   1. every lane p < P bounds "its" sub-bucket against the new sample and the warp ballots the buckets to visit;
-    //   2. visited buckets only (a handful out of n/32 after the first few hundred samples) are updated through a
-    //      switch over the set bits -- the running minima live in registers, so the index must be static, and an
-    //      unrolled `if (mask >> p & 1)` ladder costs ~40 cycles per bucket even when nothing is visited;
+    //   2. visited buckets only (a handful out of n/32 after the first few hundred samples) are updated, one generic
+    //      body per set bit of the ballot, their running minima loaded and stored at a dynamic TMEM column (or shared
+    //      memory slot);
     //   3. warp arg-max over the P bucket summaries, one 16-byte slot per warp (value, ~rank, sorted position of the
     //      bucket's best point), one barrier, arg-max over the 16 slots.  The winner's SORTED POSITION travels with the
     //      slot, so the next iteration reads its coordinates directly (no index -> position lookup on the chain).
@@ -411,11 +365,12 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
     if (CL) {
         if (tid < 64) cslot[tid >> 5][tid & 31] = make_uint4(0u, 0u, 0u, 0u);
         if (tid == 0) {
-            xbar_init(&xbar[0]);
-            xbar_init(&xbar[1]);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            xbar_arm(&xbar[0], csize * 32u);   // each phase receives one 32-byte record from every CTA of the cluster
-            xbar_arm(&xbar[1], csize * 32u);
+            mbar_init(smem_u32(&xbar[0]), 1);
+            mbar_init(smem_u32(&xbar[1]), 1);
+            mbar_init_fence();
+            // the one local arrival + the bytes a phase receives: one 32-byte record from every CTA of the cluster
+            mbar_expect_tx(smem_u32(&xbar[0]), csize * 32u);
+            mbar_expect_tx(smem_u32(&xbar[1]), csize * 32u);
         }
     }
     __syncthreads();
@@ -433,25 +388,6 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
     unsigned long long visited = 0;
     uint32_t wm = 0u, wr = 0u, wpos = 0u;   // this warp's best (value, ~rank, position): recomputed only after a visit
 
-#define SPSK_FPS_BUCKET(PP)                                                                                      \
-    case PP:                                                                                                     \
-        if (PP < P) {                                                                                            \
-            const int pos = (PP * W + warp) * 32 + lane;                                                         \
-            const float d = sqdist3(sx[pos], sy[pos], sz[pos], x1, y1, z1);                                      \
-            const float t = fminf(d, tmp[(!GEN && PP < P) ? PP : 0]);                                            \
-            tmp[(!GEN && PP < P) ? PP : 0] = t;                                                                  \
-            const uint32_t oi = oidx[PP < P ? PP : 0];                                                           \
-            const bool valid = oi != 0xFFFFFFFFu;                                                                \
-            const uint32_t u = (valid && t > 0.f) ? __float_as_uint(t) : 0u;                                     \
-            const uint32_t mx = __reduce_max_sync(0xFFFFFFFFu, u);                                               \
-            const uint32_t cand = (valid && u == mx) ? ~fps_rank(oi, s_mask, s_log2) : 0u;                       \
-            const uint32_t rr = __reduce_max_sync(0xFFFFFFFFu, cand);                                            \
-            uint32_t bp = 0u;   /* cluster mode only: the best point's position travels with the summary */      \
-            if (CL) bp = __reduce_max_sync(0xFFFFFFFFu, (valid && cand == rr) ? (uint32_t)pos : 0u);             \
-            if (lane == PP) { bmax_bits = mx; brank = rr; bpos = bp; }                                           \
-        }                                                                                                        \
-        break;
-
     for (int j = 1; j < m; ++j) {
         long long t0 = (PROF && pf) ? clock64() : 0;
         const float x1 = CL ? qx : sx[qpos], y1 = CL ? qy : sy[qpos], z1 = CL ? qz : sz[qpos];
@@ -461,78 +397,36 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
         const float lz = fmaxf(fmaxf(__fsub_rn(bz0, z1), __fsub_rn(z1, bz1)), 0.f);
         const float lb = __fmaf_rn(lz, lz, __fmaf_rn(lx, lx, __fmul_rn(ly, ly)));
         const bool act = (lane < P) && (lb < __uint_as_float(bmax_bits));
-        uint32_t mask = __ballot_sync(0xFFFFFFFFu, act);
-        const uint32_t mask0 = mask;
+        const uint32_t mask = __ballot_sync(0xFFFFFFFFu, act);
         if (PROF && pf) { const long long t1 = clock64(); pc[0] += t1 - t0; t0 = t1; }
         if (PROF && prof != nullptr && lane == 0) visited += __popc(mask);
-#define SPSK_FPS_ALL_BUCKETS                                                                                              \
-    SPSK_FPS_BUCKET(0) SPSK_FPS_BUCKET(1) SPSK_FPS_BUCKET(2) SPSK_FPS_BUCKET(3) SPSK_FPS_BUCKET(4) SPSK_FPS_BUCKET(5)        \
-    SPSK_FPS_BUCKET(6) SPSK_FPS_BUCKET(7) SPSK_FPS_BUCKET(8) SPSK_FPS_BUCKET(9) SPSK_FPS_BUCKET(10) SPSK_FPS_BUCKET(11)      \
-    SPSK_FPS_BUCKET(12) SPSK_FPS_BUCKET(13) SPSK_FPS_BUCKET(14) SPSK_FPS_BUCKET(15) SPSK_FPS_BUCKET(16) SPSK_FPS_BUCKET(17)  \
-    SPSK_FPS_BUCKET(18) SPSK_FPS_BUCKET(19) SPSK_FPS_BUCKET(20) SPSK_FPS_BUCKET(21) SPSK_FPS_BUCKET(22) SPSK_FPS_BUCKET(23)  \
-    SPSK_FPS_BUCKET(24) SPSK_FPS_BUCKET(25) SPSK_FPS_BUCKET(26) SPSK_FPS_BUCKET(27) SPSK_FPS_BUCKET(28) SPSK_FPS_BUCKET(29)  \
-    SPSK_FPS_BUCKET(30) SPSK_FPS_BUCKET(31)
-        if (GEN) {
-            // generic body, dynamic sub-bucket index: the running minimum and the point's tie-break key come from TMEM (or
-            // shared memory)
-            uint32_t mk = mask;
-            while (mk) {
-                const int pb = __ffs(mk) - 1;
-                mk &= mk - 1u;
-                const int pos = (pb * W + warp) * 32 + lane;
-                uint32_t tb, ir;
-                if (TM) tmem_ld_x2(tbase + 2u * (uint32_t)pb, tb, ir);
-                else { tb = __float_as_uint(stmp[pos]); ir = sir[pos]; }
-                const float d = sqdist3(sx[pos], sy[pos], sz[pos], x1, y1, z1);
-                const float t = fminf(d, __uint_as_float(tb));
-                if (TM) tmem_st_x1(tbase + 2u * (uint32_t)pb, __float_as_uint(t));
-                else stmp[pos] = t;
-                const uint32_t u = (t > 0.f) ? __float_as_uint(t) : 0u;   // padding keeps t = -1, ir = 0
-                const uint32_t mx = __reduce_max_sync(0xFFFFFFFFu, u);
-                const uint32_t cand = (u == mx) ? ir : 0u;
-                const uint32_t rr = __reduce_max_sync(0xFFFFFFFFu, cand);
-                uint32_t bp = 0u;   // cluster mode only: the best point's position travels with the summary
-                if (CL) bp = __reduce_max_sync(0xFFFFFFFFu, (ir != 0u && cand == rr) ? (uint32_t)pos : 0u);
-                if (lane == pb) { bmax_bits = mx; brank = rr; bpos = bp; }
-            }
-            // (the tcgen05.wait::st that orders these stores before the next load of the same columns -- a later iteration -- is
-            // taken after the block barrier below, off the critical warp's path to it)
-        } else if (LADDER == 2) {
-            // two-level ladder: groups of 8 sub-buckets, then the bits of a non-empty group
-#pragma unroll
-            for (int g = 0; g < P; g += 8) {
-                if ((mask >> g) & 0xFFu) {
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const int pb = g + q;
-                        if (pb < P && ((mask >> pb) & 1u)) {
-                            switch (pb) { SPSK_FPS_ALL_BUCKETS default: break; }
-                        }
-                    }
-                }
-            }
-        } else if (LADDER == 1) {
-            // few sub-buckets per warp: a straight ladder of bit tests (the switch below costs an indirect branch per visit)
-            if (mask) {
-#pragma unroll
-                for (int pb = 0; pb < P; ++pb) {
-                    if ((mask >> pb) & 1u) {
-                        switch (pb) { SPSK_FPS_ALL_BUCKETS default: break; }
-                    }
-                }
-            }
-        } else {
-            while (mask) {
-                const int pb = __ffs(mask) - 1;
-                mask &= mask - 1u;
-                switch (pb) { SPSK_FPS_ALL_BUCKETS default: break; }
-            }
+        // visit: the running minimum and the point's tie-break key come from TMEM (or shared memory)
+        uint32_t mk = mask;
+        while (mk) {
+            const int pb = __ffs(mk) - 1;
+            mk &= mk - 1u;
+            const int pos = (pb * W + warp) * 32 + lane;
+            uint32_t tb, ir;
+            if (TM) tmem_ld_x2(tbase + 2u * (uint32_t)pb, tb, ir);
+            else { tb = __float_as_uint(stmp[pos]); ir = sir[pos]; }
+            const float d = sqdist3(sx[pos], sy[pos], sz[pos], x1, y1, z1);
+            const float t = fminf(d, __uint_as_float(tb));
+            if (TM) tmem_st_x1(tbase + 2u * (uint32_t)pb, __float_as_uint(t));
+            else stmp[pos] = t;
+            const uint32_t u = (t > 0.f) ? __float_as_uint(t) : 0u;   // padding keeps t = -1, ir = 0
+            const uint32_t mx = __reduce_max_sync(0xFFFFFFFFu, u);
+            const uint32_t cand = (u == mx) ? ir : 0u;
+            const uint32_t rr = __reduce_max_sync(0xFFFFFFFFu, cand);
+            uint32_t bp = 0u;   // cluster mode only: the best point's position travels with the summary
+            if (CL) bp = __reduce_max_sync(0xFFFFFFFFu, (ir != 0u && cand == rr) ? (uint32_t)pos : 0u);
+            if (lane == pb) { bmax_bits = mx; brank = rr; bpos = bp; }
         }
-#undef SPSK_FPS_ALL_BUCKETS
+        // (the tcgen05.wait::st that orders these stores before the next load of the same columns -- a later iteration -- is
+        // taken after the block barrier below, off the critical warp's path to it)
         if (PROF && pf) { const long long t1 = clock64(); pc[1] += t1 - t0; t0 = t1; }
         // warp best over its P sub-buckets: unchanged (cached) when this warp visited nothing -- most warps, most iterations;
         // their REDUX would only compete with the critical warp's for the same unit
-        if (mask0) {
+        if (mask) {
             const uint32_t wv = (lane < P) ? bmax_bits : 0u;
             wm = __reduce_max_sync(0xFFFFFFFFu, wv);
             const uint32_t wc = (lane < P && bmax_bits == wm) ? brank : 0u;
@@ -547,7 +441,7 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
             }
             if (PROF && pf) { const long long t1 = clock64(); pc[2] += t1 - t0; t0 = t1; }
             __syncthreads();
-            if (TM && mask0) tmem_wait_st();
+            if (TM && mask) tmem_wait_st();
             if (PROF && pf) { const long long t1 = clock64(); pc[3] += t1 - t0; t0 = t1; }
             // block best over the W warp slots
             const uint2 v = sl[lane];
@@ -556,9 +450,8 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
             // the barrier on every warp and VOTE + SHFL are no faster than one REDUX)
             const uint32_t m2 = __reduce_max_sync(0xFFFFFFFFu, v.x);
             const uint32_t r2 = __reduce_max_sync(0xFFFFFFFFu, (v.x == m2) ? v.y : 0u);
-            // the sample's original index: rank(k) = brev(k & s_mask) | (k >> s_log2); its sorted position through the map
-            const uint32_t rank = ~r2;
-            const int old = (int)((__brev(rank) & s_mask) | ((rank & ((1u << (32u - s_log2)) - 1u)) << s_log2));
+            // the sample's original index; its sorted position through the map
+            const int old = (int)fps_unrank(~r2, s_mask, s_log2);
             qpos = pos_of[old];
             if (warp == 0) {
                 if (lane == (j & 31)) keep = old;
@@ -570,7 +463,7 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
             uint4 *cs_ = cslot[j & 1];
             if (lane == 0) cs_[warp] = make_uint4(wm, wr, wpos, 0u);
             __syncthreads();
-            if (TM && mask0) tmem_wait_st();
+            if (TM && mask) tmem_wait_st();
             const uint4 sv = cs_[lane];
             const uint32_t cm = __reduce_max_sync(0xFFFFFFFFu, sv.x);
             const uint32_t cr = __reduce_max_sync(0xFFFFFFFFu, (sv.x == cm) ? sv.y : 0u);
@@ -599,15 +492,13 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
             // 4. re-arm this table's barrier for its next phase (iteration j + 2).  Safe to do as soon as this thread has passed
             //    the wait: no CTA can send iteration j + 2 before it has received OUR record of iteration j + 1, which is sent
             //    after this point; a slower warp of this CTA still waiting on the old parity sees it as completed.
-            if (tid == 0) xbar_arm(xb, csize * 32u);
+            if (tid == 0) mbar_expect_tx(smem_u32(xb), csize * 32u);
             if (crank == 0 && warp == 0) {
-                const uint32_t rank = ~w0.y;
-                if (lane == (j & 31)) keep = (int)((__brev(rank) & s_mask) | ((rank & ((1u << (32u - s_log2)) - 1u)) << s_log2));
+                if (lane == (j & 31)) keep = (int)fps_unrank(~w0.y, s_mask, s_log2);
                 if ((j & 31) == 31) idx[j - 31 + lane] = keep;
             }
         }
     }
-#undef SPSK_FPS_BUCKET
     if (crank == 0 && warp == 0 && (m & 31) != 0 && lane < (m & 31)) idx[(m & ~31) + lane] = keep;   // the last partial line
     if (PROF && prof != nullptr) {
         if (pf) for (int i = 0; i < 5; ++i) atomicAdd(prof + i, pc[i]);
@@ -616,15 +507,10 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
     if (temp) {
 #pragma unroll
         for (int p = 0; p < P; ++p) {
-            if (GEN) {
-                uint32_t tb, ir;
-                if (TM) tmem_ld_x2(tbase + 2u * p, tb, ir);
-                else { const int pos = (p * W + warp) * 32 + lane; tb = __float_as_uint(stmp[pos]); ir = sir[pos]; }
-                const uint32_t rank = ~ir;   // rank(k) = brev(k & s_mask) | (k >> s_log2): the point's scene index, recovered
-                if (ir != 0u) temp[(__brev(rank) & s_mask) | ((rank & ((1u << (32u - s_log2)) - 1u)) << s_log2)] = __uint_as_float(tb);
-            } else if (oidx[p] != 0xFFFFFFFFu) {
-                temp[oidx[p]] = tmp[(!GEN) ? p : 0];
-            }
+            uint32_t tb, ir;
+            if (TM) tmem_ld_x2(tbase + 2u * p, tb, ir);
+            else { const int pos = (p * W + warp) * 32 + lane; tb = __float_as_uint(stmp[pos]); ir = sir[pos]; }
+            if (ir != 0u) temp[fps_unrank(~ir, s_mask, s_log2)] = __uint_as_float(tb);   // ~rank gives back the scene index
         }
     }
     if (TM) {
@@ -635,69 +521,25 @@ fps_pruned_kernel(int n_scene, int m, const float *__restrict__ src, float *__re
 }
 
 static unsigned long long *g_fps_prof = nullptr;
-constexpr int SPSK_FPS_NO_CLUSTER = 1;   // internal: the requested cluster size cannot run here, use the streaming kernel
 
-template <int P, bool CL, int LADDER, bool PROF = false, int ST = 0>
-static int launch_fps_pruned_v(int b, int n, int m, int csize, const float *src, float *temp, int *idx, cudaStream_t st) {
-    const size_t smem = sizeof(float) * 3 * 512 * P + (CL ? 0 : sizeof(unsigned short) * 512 * P)   // xyz (+ index -> position map)
-                        + (ST == 2 ? 8 * 512 * P : 0);                                               // (+ minima and ~rank)
-    auto kern = fps_pruned_kernel<P, CL, LADDER, PROF, ST>;
-    static const int bitonic = getenv("SPSK_FPS_SORT") != nullptr && getenv("SPSK_FPS_SORT")[0] == 'b' ? 1 : 0;   // A/B: the round-1 full sort
-    if (smem + 8192 > 48 * 1024) {
-        static SmemAttrOnce attr;   // one static per template instantiation: set once per (kernel, device), not per launch
-        if (int rc = attr.ensure(reinterpret_cast<const void *>(kern), (int)smem, "cudaFuncSetAttribute(fps_pruned_kernel)")) return rc;
-    }
-    if (!CL) {
-        kern<<<b, 512, smem, st>>>(n, m, src, temp, idx, g_fps_prof, bitonic);
-    } else {
-        if (csize > 8) {
-            // 16-CTA clusters are a non-portable size: opt in, and make sure this device can co-schedule one
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            if (e != cudaSuccess) { (void)cudaGetLastError(); return SPSK_FPS_NO_CLUSTER; }
-        }
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(b * csize));
-        cfg.blockDim = dim3(512);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)csize;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        if (csize > 8) {
-            int nclusters = 0;
-            cudaError_t q = cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg);
-            if (q != cudaSuccess || nclusters < 1) { (void)cudaGetLastError(); return SPSK_FPS_NO_CLUSTER; }
-        }
-        cudaError_t e = cudaLaunchKernelEx(&cfg, kern, n, m, src, temp, idx, g_fps_prof, bitonic);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaLaunchKernelEx(fps_pruned_kernel, cluster)");
-    }
-    SPSK_LAUNCH_CHECK("fps_pruned_kernel");
-    return SPSK_OK;
-}
-
-// bucket dispatch: ladder of bit tests for few sub-buckets per warp, switch over the set bits for many
-// (SPSK_FPS_DISPATCH=ladder|switch overrides, for A/B measurements)
+// csize: CTAs per scene (CL only).  Returns SPSK_CLUSTER_UNSCHEDULABLE when the device cannot co-schedule such a cluster.
 template <int P, bool CL>
 static int launch_fps_pruned(int b, int n, int m, int csize, const float *src, float *temp, int *idx, cudaStream_t st) {
-    // P >= 16 (n > 4096 points per CTA): running minima in tensor memory, generic visit loop (see the kernel).  These CTAs fill
-    // their SM's shared memory, so the TMEM columns they hold never compete with a co-resident tensor-core kernel; the smaller
-    // shapes (short ladders, CTAs that share their SM with sa_mma CTAs wanting all 512 columns) keep the register kernel.
-    static const bool no_tm = getenv("SPSK_FPS_NOTMEM") != nullptr;   // A/B and fallback: the round-1 register kernel everywhere
-    if (!no_tm) {
-        constexpr int ST = P >= 16 ? 1 : 2;
-        if (g_fps_prof != nullptr) return launch_fps_pruned_v<P, CL, 2, true, ST>(b, n, m, csize, src, temp, idx, st);
-        return launch_fps_pruned_v<P, CL, 2, false, ST>(b, n, m, csize, src, temp, idx, st);
+    const size_t smem = sizeof(float) * 3 * 512 * P + (CL ? 0 : sizeof(unsigned short) * 512 * P)   // xyz (+ index -> position map)
+                        + (P >= 16 ? 0 : 8 * 512 * P);                                               // (+ minima and ~rank)
+    const bool prof = g_fps_prof != nullptr;
+    auto kern = prof ? fps_pruned_kernel<P, CL, true> : fps_pruned_kernel<P, CL, false>;
+    if constexpr (CL) {
+        static ClusterKernelState state[2];   // one per kernel: [prof]
+        return launch_cluster(state[prof], kern, "fps_pruned_kernel", b, csize, 512, smem, st, n, m, src, temp, idx, g_fps_prof);
     }
-    // 1 = ladder, 2 = two-level ladder (fastest at every P on B200), 0 = switch over set bits (A/B knob of the register kernel)
-    static const int mode = [] { const char *e = getenv("SPSK_FPS_DISPATCH"); return !e ? 2 : (e[0] == 'l' ? 1 : (e[0] == 'g' ? 2 : 0)); }();
-    if (mode == 1) return launch_fps_pruned_v<P, CL, 1>(b, n, m, csize, src, temp, idx, st);
-    if (mode == 2 && g_fps_prof != nullptr) return launch_fps_pruned_v<P, CL, 2, true>(b, n, m, csize, src, temp, idx, st);
-    if (mode == 2) return launch_fps_pruned_v<P, CL, 2>(b, n, m, csize, src, temp, idx, st);
-    return launch_fps_pruned_v<P, CL, 0>(b, n, m, csize, src, temp, idx, st);
+    if (smem + 8192 > 48 * 1024) {
+        static SmemAttrOnce attr[2];   // one per kernel: [prof]
+        if (int rc = attr[prof].ensure(reinterpret_cast<const void *>(kern), (int)smem, "cudaFuncSetAttribute(fps_pruned_kernel)")) return rc;
+    }
+    kern<<<b, 512, smem, st>>>(n, m, src, temp, idx, g_fps_prof);
+    SPSK_LAUNCH_CHECK("fps_pruned_kernel");
+    return SPSK_OK;
 }
 
 // Small scenes, n < 1024: the reference block has S = 2^floor(log2 n) < 1024 threads; T = blockDim.x =
@@ -874,22 +716,14 @@ static int fps_dispatch(int b, int n, int m, const float *src, float *temp, int 
     const int threads = S < 32 ? 32 : S;  // multiple of S, >= one warp; 1024 for n >= 1024
     const int per_thread = (n + threads - 1) / threads;
     const bool fits = per_thread <= 16;  // 16 x 1024 padded points of SoA xyz = 192 KB of shared memory
-    // n > 16384 (Waymo-shaped scenes): one 8-CTA cluster per scene, each CTA prunes its own slice, DSMEM arg-max
-    // cluster size: the fewest CTAs that hold the scene (16384 points each) -- least SM-time per scene, which is what a
-    // pipelined serving loop pays; SPSK_FPS_CLUSTER=8 trades SMs for latency
-    // 131072 < n <= 262144: one 16-CTA cluster (non-portable size; falls through to the streaming kernel if the device
-    // cannot co-schedule it)
+    // n > 16384 (Waymo-shaped scenes): one cluster per scene, each CTA prunes its own slice, DSMEM arg-max.  Cluster size: the
+    // fewest CTAs that hold the scene -- least SM-time per scene, which is what a pipelined serving loop pays.  n <= 16384 * cl,
+    // so a CTA owns at most 16384 points: the P = 32 kernel holds them.  131072 < n <= 262144 takes a 16-CTA cluster
+    // (non-portable size; falls through to the streaming kernel if the device cannot co-schedule it).
     if (!DISTMAT && threads == 1024 && n > 16384 && n <= 16 * 16384 && !fps_dense_forced()) {
-        int cl = n <= 2 * 16384 ? 2 : (n <= 4 * 16384 ? 4 : (n <= 8 * 16384 ? 8 : 16));
-        static const int want_cl = [] { const char *e = getenv("SPSK_FPS_CLUSTER"); return e ? atoi(e) : 0; }();
-        if ((want_cl == 2 || want_cl == 4 || want_cl == 8 || want_cl == 16) && want_cl >= cl) cl = want_cl;
-        const int per_cta = (n + cl - 1) / cl;
-        int rc;
-        if (per_cta <= 2048) rc = launch_fps_pruned<4, true>(b, n, m, cl, src, temp, idx, st);
-        else if (per_cta <= 4096) rc = launch_fps_pruned<8, true>(b, n, m, cl, src, temp, idx, st);
-        else if (per_cta <= 8192) rc = launch_fps_pruned<16, true>(b, n, m, cl, src, temp, idx, st);
-        else rc = launch_fps_pruned<32, true>(b, n, m, cl, src, temp, idx, st);
-        if (rc != SPSK_FPS_NO_CLUSTER) return rc;
+        const int cl = n <= 2 * 16384 ? 2 : (n <= 4 * 16384 ? 4 : (n <= 8 * 16384 ? 8 : 16));
+        const int rc = launch_fps_pruned<32, true>(b, n, m, cl, src, temp, idx, st);
+        if (rc != SPSK_CLUSTER_UNSCHEDULABLE) return rc;
     }
     if (!fits) {
         SPSK_REQUIRE(temp != nullptr, SPSK_ERR_UNSUPPORTED,

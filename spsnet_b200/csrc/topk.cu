@@ -134,43 +134,12 @@ static int launch_score_topk_cluster(int b, int n, int n_pad, int num_class, int
                                      int *idx, float *scores, cudaStream_t st) {
     const int csize = n_pad / TOPK_CTA_KEYS;
     const size_t smem = sizeof(unsigned long long) * TOPK_CTA_KEYS;
-    auto kern = score_topk_cluster_kernel;
-    static SmemAttrOnce attr;
-    if (int rc = attr.ensure(reinterpret_cast<const void *>(kern), (int)smem, "cudaFuncSetAttribute(score_topk_cluster_kernel)")) return rc;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(b * csize));
-    cfg.blockDim = dim3(TOPK_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute cl[1];
-    cl[0].id = cudaLaunchAttributeClusterDimension;
-    cl[0].val.clusterDim.x = (unsigned)csize;
-    cl[0].val.clusterDim.y = 1;
-    cl[0].val.clusterDim.z = 1;
-    cfg.attrs = cl;
-    cfg.numAttrs = 1;
-    if (csize > 8) {
-        // 16-CTA clusters are a non-portable size: opt in, and make sure this device can co-schedule one.  The answer cannot
-        // change for a (kernel, device), so it is asked once per device (and never again inside a CUDA-graph capture).
-        static signed char schedulable[64] = {};   // 0 = not asked yet, 1 = yes, -1 = no
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
-        if (schedulable[dev] == 0) {
-            int nclusters = 0;
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            if (e == cudaSuccess) e = cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg);
-            if (e != cudaSuccess) (void)cudaGetLastError();
-            schedulable[dev] = e == cudaSuccess && nclusters >= 1 ? 1 : -1;
-        }
-        if (schedulable[dev] < 0) {
-            set_error("score_topk: n=%d needs a 16-CTA cluster of %zu-byte CTAs, which this device cannot schedule", n, smem);
-            return SPSK_ERR_UNSUPPORTED;
-        }
-    }
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, n, n_pad, num_class, npoint, cls, stds, idx, scores);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaLaunchKernelEx(score_topk_cluster_kernel)");
-    SPSK_LAUNCH_CHECK("score_topk_cluster_kernel");
-    return SPSK_OK;
+    static ClusterKernelState state;
+    const int rc = launch_cluster(state, score_topk_cluster_kernel, "score_topk_cluster_kernel", b, csize, TOPK_THREADS, smem, st,
+                                  n, n_pad, num_class, npoint, cls, stds, idx, scores);
+    SPSK_REQUIRE(rc != SPSK_CLUSTER_UNSCHEDULABLE, SPSK_ERR_UNSUPPORTED,
+                 "score_topk: n=%d needs a 16-CTA cluster of %zu-byte CTAs, which this device cannot schedule", n, smem);
+    return rc;
 }
 
 }  // namespace spsk

@@ -171,7 +171,9 @@ SPSK_API int spsk_ball_query_msg(int b, int n, int m, int nscales, const float *
  * edge >= 1.01 * max radius, 3 x 3 neighbourhood per centre, hits ordered through a per-warp index bitmap):
  * the work drops from n to a few dozen pair tests per centre when the radius is small against the scene.
  * `workspace` is caller-owned device scratch of at least spsk_ball_query_grid_workspace_bytes(b, n) bytes.
- * n <= 65536. */
+ * n <= SPSK_BQ_GRID_MAX_N (SPSK_ERR_UNSUPPORTED above): the grid is built per window of 65536 point ids and the
+ * query walks windows of 65536 ids (32768 with four scales) in increasing id order until every scale is full. */
+#define SPSK_BQ_GRID_MAX_N 262144
 SPSK_API long long spsk_ball_query_grid_workspace_bytes(int b, int n);
 SPSK_API int spsk_ball_query_msg_grid(int b, int n, int m, int nscales, const float *radius, const int *nsample,
                              const float *new_xyz, const float *xyz, int *const *idx, void *workspace,

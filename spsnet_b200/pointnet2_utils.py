@@ -268,6 +268,10 @@ class BallQuery(Function):
         _chk(xyz, "xyz", torch.float32, 3)
         B, N, _ = xyz.shape
         npoint = new_xyz.shape[1]
+        if GRID_BQ_MIN_N < N <= GRID_MAX_N:
+            # the brute-force scan reads all N points for every centre whose ball holds fewer than nsample of them; the grid
+            # kernel writes empty rows as zeros, which is what the zero-filled output below would hold
+            return ball_query_msg([radius], [nsample], xyz, new_xyz, grid=True)[0]
         idx = torch.zeros((B, npoint, nsample), dtype=torch.int32, device=xyz.device)
         with torch.cuda.device(xyz.device):
             check(lib.spsk_ball_query(B, N, npoint, float(radius), int(nsample), new_xyz.data_ptr(), xyz.data_ptr(),
@@ -397,12 +401,14 @@ def gather_rows(points: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
 
 
 GRID_MIN_N = 2048  # below this the brute-force scan (early exit, smem tiles) is as fast as building a grid
+GRID_MAX_N = 262144  # include/spsk.h: SPSK_BQ_GRID_MAX_N
+GRID_BQ_MIN_N = 65536  # BallQuery (single radius) takes the grid kernel above this many points
 
 
 def ball_query_msg(radii, nsamples, xyz: torch.Tensor, new_xyz: torch.Tensor, grid=None):
     """All scales of an MSG layer in ONE pass; returns a list of (B, npoint, nsample_s) int32 tensors,
     identical to [ball_query(r, ns, xyz, new_xyz) for r, ns in zip(radii, nsamples)].  grid=None picks the
-    uniform-grid kernel for n >= GRID_MIN_N and the brute-force scan otherwise (same results)."""
+    uniform-grid kernel for GRID_MIN_N <= n <= GRID_MAX_N and the brute-force scan otherwise (same results)."""
     _chk(new_xyz, "new_xyz", torch.float32, 3)
     _chk(xyz, "xyz", torch.float32, 3)
     S = len(radii)
@@ -412,10 +418,7 @@ def ball_query_msg(radii, nsamples, xyz: torch.Tensor, new_xyz: torch.Tensor, gr
     r = (C.c_float * S)(*[float(x) for x in radii])
     n = (C.c_int * S)(*[int(x) for x in nsamples])
     ptrs = (C.c_void_p * S)(*[o.data_ptr() for o in outs])
-    # the grid kernel keeps 8 per-warp hit bitmaps of S * ceil(N / 32) words in shared memory (ball_query_grid.cu): auto-select it
-    # only while they fit its 200 KB budget, else the brute-force scan (same results)
-    grid_fits = 8 * S * ((N + 31) // 32) * 4 <= 200 * 1024
-    use_grid = (GRID_MIN_N <= N <= 65536 and grid_fits) if grid is None else bool(grid)
+    use_grid = (GRID_MIN_N <= N <= GRID_MAX_N) if grid is None else bool(grid)
     with torch.cuda.device(xyz.device):
         if use_grid:
             nbytes = int(lib.spsk_ball_query_grid_workspace_bytes(B, N))

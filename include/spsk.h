@@ -109,7 +109,15 @@ SPSK_API int spsk_group_points_grad(int b, int c, int n, int npoints, int nsampl
 
 /* Three nearest known points of every unknown point: squared distances (the python layer takes the
  * sqrt) and indices, first index wins ties.  Replaces three_nn_wrapper (src/interpolate.cpp:21-30
- * -> src/interpolate_gpu.cu:16-81).  unknown (b,n,3), known (b,m,3), dist2/idx (b,n,3). */
+ * -> src/interpolate_gpu.cu:16-81).  unknown (b,n,3), known (b,m,3), dist2/idx (b,n,3).
+ * Kernel choice: n >= SPSK_THREE_NN_GRID_MIN_N and SPSK_THREE_NN_GRID_MIN_M <= m <= SPSK_THREE_NN_GRID_MAX_M runs the
+ * grid kernel (one launch: each cluster of 1-16 CTAs holds a scene's known points in shared memory, sorted into xy cells,
+ * and searches rings of cells around each unknown point); every other shape runs the all-pairs kernel.  Both give
+ * bit-identical dist2 and idx: the three smallest (d, index) pairs with d < +inf, +inf / index 0 in unfilled slots.
+ * Where the device cannot schedule a 16-CTA cluster the all-pairs kernel runs instead. */
+#define SPSK_THREE_NN_GRID_MIN_N 1024
+#define SPSK_THREE_NN_GRID_MIN_M 1024
+#define SPSK_THREE_NN_GRID_MAX_M 131072
 SPSK_API int spsk_three_nn(int b, int n, int m, const float *unknown, const float *known, float *dist2,
                   int *idx, spsk_stream_t stream);
 

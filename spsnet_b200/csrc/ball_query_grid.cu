@@ -45,11 +45,6 @@ static size_t grid_ws_bytes(int b, int n) {
            sizeof(float4) * (size_t)b * n + 256;
 }
 
-__device__ __forceinline__ int cell_coord(float v, float vmin, float inv_c, int g) {
-    const int c = (int)floorf((v - vmin) * inv_c);
-    return min(max(c, 0), g - 1);
-}
-
 __global__ void __launch_bounds__(1024, 1)
 bq_grid_build_kernel(int n, float rmax, const float *__restrict__ xyz, GridParams *__restrict__ params,
                      int *__restrict__ cell_start, float4 *__restrict__ sorted) {
@@ -60,25 +55,10 @@ bq_grid_build_kernel(int n, float rmax, const float *__restrict__ xyz, GridParam
     const int win = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const float *pts = xyz + (size_t)b * n * 3;
     const int w0 = win * BG_WIN, nw = min(BG_WIN, n - w0);   // this CTA's ids [w0, w0 + nw)
-    float x0 = 3.0e38f, x1 = -3.0e38f, y0 = 3.0e38f, y1 = -3.0e38f, z0 = 3.0e38f, z1 = -3.0e38f;
-    for (int i = tid; i < n; i += 1024) {
-        const float x = __ldg(pts + (size_t)i * 3), y = __ldg(pts + (size_t)i * 3 + 1), z = __ldg(pts + (size_t)i * 3 + 2);
-        x0 = fminf(x0, x); x1 = fmaxf(x1, x); y0 = fminf(y0, y); y1 = fmaxf(y1, y); z0 = fminf(z0, z); z1 = fmaxf(z1, z);
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        x0 = fminf(x0, __shfl_xor_sync(0xFFFFFFFFu, x0, o)); x1 = fmaxf(x1, __shfl_xor_sync(0xFFFFFFFFu, x1, o));
-        y0 = fminf(y0, __shfl_xor_sync(0xFFFFFFFFu, y0, o)); y1 = fmaxf(y1, __shfl_xor_sync(0xFFFFFFFFu, y1, o));
-        z0 = fminf(z0, __shfl_xor_sync(0xFFFFFFFFu, z0, o)); z1 = fmaxf(z1, __shfl_xor_sync(0xFFFFFFFFu, z1, o));
-    }
-    if (lane == 0) { red[0][warp] = x0; red[1][warp] = x1; red[2][warp] = y0; red[3][warp] = y1; red[4][warp] = z0; red[5][warp] = z1; }
     for (int i = tid; i < BG_MAXC; i += 1024) cnt[i] = 0;
-    __syncthreads();
-    x0 = red[0][0]; x1 = red[1][0]; y0 = red[2][0]; y1 = red[3][0]; z0 = red[4][0]; z1 = red[5][0];
-    for (int w = 1; w < 32; ++w) {
-        x0 = fminf(x0, red[0][w]); x1 = fmaxf(x1, red[1][w]); y0 = fminf(y0, red[2][w]); y1 = fmaxf(y1, red[3][w]);
-        z0 = fminf(z0, red[4][w]); z1 = fmaxf(z1, red[5][w]);
-    }
+    float box[6];
+    block_box3(pts, 0, n, red, box);
+    const float x0 = box[0], x1 = box[1], y0 = box[2], y1 = box[3], z0 = box[4], z1 = box[5];
     const float ex = fmaxf(x1 - x0, 0.f), ey = fmaxf(y1 - y0, 0.f), ez = fmaxf(z1 - z0, 0.f);
     float c = fmaxf(rmax * 1.01f, 1e-6f);
     c = fmaxf(c, fmaxf(ex, ey) / (float)(BG_GMAX - 2));       // never more than BG_GMAX cells per axis

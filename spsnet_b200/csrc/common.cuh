@@ -96,7 +96,41 @@ __device__ __forceinline__ uint32_t fps_unrank(uint32_t rank, uint32_t s_mask, u
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }
 
-// ---- thread-block clusters (fps.cu, topk.cu) ------------------------------------------------------
+// ---- uniform grids over a point set (ball_query_grid.cu, interpolate.cu) --------------------------------------------------
+// Cell index of coordinate v along one axis of a grid of g cells starting at vmin: a monotone function of v, clamped into
+// [0, g).  A NaN coordinate lands in cell 0.
+__device__ __forceinline__ int cell_coord(float v, float vmin, float inv_c, int g) {
+    const int c = (int)floorf((v - vmin) * inv_c);
+    return min(max(c, 0), g - 1);
+}
+
+// Exact min / max of the x, y and z coordinates of points [lo, hi) of `pts` (x, y, z interleaved), reduced by the whole
+// block (blockDim.x a multiple of 32): every thread gets box = {x0, x1, y0, y1, z0, z1}.  fminf / fmaxf skip NaN
+// coordinates; a range without a non-NaN value keeps the start values (3e38, -3e38).  red: __shared__ float[6][32].
+__device__ __forceinline__ void block_box3(const float *__restrict__ pts, int lo, int hi, float (*red)[32], float box[6]) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
+    float x0 = 3.0e38f, x1 = -3.0e38f, y0 = 3.0e38f, y1 = -3.0e38f, z0 = 3.0e38f, z1 = -3.0e38f;
+    for (int i = lo + tid; i < hi; i += blockDim.x) {
+        const float x = __ldg(pts + (size_t)i * 3), y = __ldg(pts + (size_t)i * 3 + 1), z = __ldg(pts + (size_t)i * 3 + 2);
+        x0 = fminf(x0, x); x1 = fmaxf(x1, x); y0 = fminf(y0, y); y1 = fmaxf(y1, y); z0 = fminf(z0, z); z1 = fmaxf(z1, z);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        x0 = fminf(x0, __shfl_xor_sync(0xFFFFFFFFu, x0, o)); x1 = fmaxf(x1, __shfl_xor_sync(0xFFFFFFFFu, x1, o));
+        y0 = fminf(y0, __shfl_xor_sync(0xFFFFFFFFu, y0, o)); y1 = fmaxf(y1, __shfl_xor_sync(0xFFFFFFFFu, y1, o));
+        z0 = fminf(z0, __shfl_xor_sync(0xFFFFFFFFu, z0, o)); z1 = fmaxf(z1, __shfl_xor_sync(0xFFFFFFFFu, z1, o));
+    }
+    if (lane == 0) { red[0][warp] = x0; red[1][warp] = x1; red[2][warp] = y0; red[3][warp] = y1; red[4][warp] = z0; red[5][warp] = z1; }
+    __syncthreads();
+    x0 = red[0][0]; x1 = red[1][0]; y0 = red[2][0]; y1 = red[3][0]; z0 = red[4][0]; z1 = red[5][0];
+    for (int w = 1; w < nwarps; ++w) {
+        x0 = fminf(x0, red[0][w]); x1 = fmaxf(x1, red[1][w]); y0 = fminf(y0, red[2][w]); y1 = fmaxf(y1, red[3][w]);
+        z0 = fminf(z0, red[4][w]); z1 = fmaxf(z1, red[5][w]);
+    }
+    box[0] = x0; box[1] = x1; box[2] = y0; box[3] = y1; box[4] = z0; box[5] = z1;
+}
+
+// ---- thread-block clusters (fps.cu, topk.cu, interpolate.cu) --------------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ uint32_t cluster_nctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {

@@ -191,6 +191,12 @@ class ThreeNN(Function):
 
 three_nn = ThreeNN.apply
 
+# include/spsk.h: spsk_three_nn runs the grid kernel for n >= THREE_NN_GRID_MIN_N and THREE_NN_GRID_MIN_M <= m <=
+# THREE_NN_GRID_MAX_M, the all-pairs kernel otherwise (bit-identical results)
+THREE_NN_GRID_MIN_N = 1024  # SPSK_THREE_NN_GRID_MIN_N
+THREE_NN_GRID_MIN_M = 1024  # SPSK_THREE_NN_GRID_MIN_M
+THREE_NN_GRID_MAX_M = 131072  # SPSK_THREE_NN_GRID_MAX_M
+
 
 class ThreeInterpolate(Function):
     """reference: pointnet2_utils.py:136-178 (ThreeInterpolate)."""
